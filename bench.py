@@ -200,13 +200,15 @@ def run_reference(args, rank, world):
     times = []
     it = 0
     while len(times) < args.steps:
-        ref.dada_uniques(seqs, ab, None, err, q, multithread=True)
+        last = ref.dada_uniques(seqs, ab, None, err, q, multithread=True)
         dt = ref.last_native_s                   # the native call alone (ctypes marshalling of 1e6 Python strings is not the reference's time)
         if it >= warm:
             times.append(dt)
         it += 1
         if times and (time.perf_counter() - t_begin) + dt > budget:
             break
+    if args.dump_outputs:
+        dump_outputs(last, args.dump_outputs)
     tsum = sum(times)
     val = args.nuniques * len(times) / tsum
     line = {"impl": "reference", "metric": "unique-reads/sec through dada()", "value": val, "unit": "uniques/s",
@@ -241,6 +243,44 @@ def measure(res, err, steps, warmup, flush, barrier, torch):
         dev_ms += last["stats"]["ms_device"]
     barrier()
     return time.perf_counter() - t0, step_ms, step_host, dev_ms, last
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+PER_UNIQUE = ("map", "pval")
+
+
+def dump_outputs(res, out_dir):
+    """Writes the arrays of one dada_uniques() result as out_dir/<field>.npy (clustering.pval.npy, map.npy, ...), all float64
+    and all finite: integers exactly, strings as rows of ASCII codes padded with 0.  A field with NaN or infinite entries
+    (the birth fields of the first cluster, which is not born by a division, are NA) holds 0 there, and
+    <field>.nonfinite.npy says which entries those are and what they were: 1 NaN, 2 +inf, 3 -inf, 0 elsewhere.  When the
+    whole set would pass 64 MB, the per-unique fields keep a fixed seeded sample of the uniques, whose indices go to
+    sample_idx.npy."""
+    from tests import cases
+    arrs = {}
+    for k, v in cases.flatten(res).items():
+        if v.dtype.kind == "U":
+            b = v.astype("S")
+            v = np.frombuffer(b.tobytes(), np.uint8).reshape(len(b), b.itemsize)
+        v = v.astype(np.float64)
+        bad = ~np.isfinite(v)
+        if bad.any():
+            arrs[k + ".nonfinite"] = np.where(np.isnan(v), 1.0, np.where(v == np.inf, 2.0, np.where(v == -np.inf, 3.0, 0.0)))
+            v = np.where(bad, 0.0, v)
+        arrs[k] = v
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_LIMIT_BYTES:
+        nraw = len(arrs["map"])
+        per_unique = [k for k in arrs if k.split(".nonfinite")[0] in PER_UNIQUE]
+        rest = total - sum(arrs[k].nbytes for k in per_unique)
+        keep = (DUMP_LIMIT_BYTES - rest) // (8 * (len(per_unique) + 1))
+        idx = np.sort(np.random.default_rng(0).choice(nraw, keep, replace=False))
+        for k in per_unique:
+            arrs[k] = arrs[k][idx]
+        arrs["sample_idx"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def selfconsist_loop(runner, n, native_s=None):
@@ -333,6 +373,9 @@ def main():
     ap.add_argument("--no-legs", action="store_true", help="N=1: skip the secondary legs (configs1, selfconsist, config5, bimera)")
     ap.add_argument("--bimera-seconds", type=int, default=60, help="N=1: timeout of the post-measurement bimera-detection leg (0 = off)")
     ap.add_argument("--watchdog", type=int, default=1700, help="dump stacks and exit after this many seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step (rank 0) as DIR/<field>.npy; the seeded inputs are the same "
+                         "in every run with the same arguments, so two builds can be compared output for output")
     args = ap.parse_args()
     import faulthandler
     faulthandler.dump_traceback_later(args.watchdog, exit=True)
@@ -431,6 +474,8 @@ def main():
     rc = 0
     if rank == 0:
         from tests import cases
+        if args.dump_outputs:
+            dump_outputs(last, args.dump_outputs)
         L = len(seqs[0])
         peak, peak_src = measured_peak_gbs()
         # ---- roofline of the dominant kernel family (CUDA-event sums per family, measured inside the library on its stream) ----

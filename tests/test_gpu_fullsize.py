@@ -1,7 +1,7 @@
 """BASELINE-size checks on the GPU (configs[1]: 1e5 synthetic 250-nt uniques): size-independent properties
-(tests/properties.py, pinned on the oracle at small sizes), run-to-run determinism, one-shot == resident, and -- when the
-reference's own C++ travelled to the box (oracle/_ref/libdada2ref.so, a few seconds on the host cores at this size) -- the full
-output against it.  bench.py diffs the 1e6 workload against the same library in its cpu_baseline leg."""
+(tests/properties.py, pinned on the oracle at small sizes), run-to-run determinism, one-shot == resident, and the output
+against the reference's own C++ on the same input (tests/golden/e2e_fullsize_1e5.npz, tools/make_golden_fuzz.py: every
+per-cluster field whole, the per-unique map / pval at a seeded sample).  bench.py diffs the 1e6 workload against the same library in its cpu_baseline leg."""
 import numpy as np
 import pytest
 
@@ -26,11 +26,10 @@ def test_1e5_uniques_invariants_determinism_and_paths_agree():
     check_invariants(seqs, ab, a)
     found = set(a["clustering"]["sequence"])
     assert len(found) == 100 and sum(v in found for v in truth["variants"]) >= 95     # the planted variants are recovered
-    from oracle import ref
-    if ref.available():                                           # the reference's C++ on the same 1e5 uniques
-        import os
-        ref.set_threads(min(16, os.cpu_count() or 1))
-        want = ref.dada_uniques(seqs, ab, None, err, q, multithread=True)
-        cases.assert_same(a, want, rtol=1e-10, label="1e5 uniques vs the reference's C++")
+    from tests.test_oracle import load_golden
+    want = load_golden("fullsize_1e5")                            # the reference's C++ on the same 1e5 uniques
+    idx = want.pop("sample_idx")
+    cases.assert_same(dict(a, map=np.asarray(a["map"])[idx], pval=np.asarray(a["pval"])[idx]), want, rtol=1e-10,
+                      label="1e5 uniques vs the reference's C++ (map / pval at %d sampled uniques)" % len(idx))
     st = a["stats"]
     assert st["gpu_launches"] > 1000 and st["n_nw"] > 1_000_000 and st["n_final_nw"] == 100000
